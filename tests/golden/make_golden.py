@@ -49,8 +49,9 @@ def rel(a, b):
     return float((a - b).norm() / b.norm().clamp_min(1e-30))
 
 
-# full-tensor gradients kept by the full-depth case (fp16 after a per-tensor max-normalisation; every bias / LayerNorm
-# vector of the model is kept whole in fp32 as well)
+# weight gradients kept by the full-depth case: GRAD_SAMPLES elements of each tensor, its first and last row plus a fixed,
+# seeded random sample (flat indices + values, fp16 after a per-tensor max-normalisation); every bias / LayerNorm vector of
+# the model is kept whole, packed the same way.  This keeps the fixture under 1 MB.
 FULL_GRAD_KEYS = (
     "vision_model.encoder.layers.11.mlp.fc1.weight", "vision_model.encoder.layers.0.self_attn.q_proj.weight",
     "vision_model.encoder.layers.0.self_attn.k_proj.weight", "vision_model.encoder.layers.0.self_attn.out_proj.weight",
@@ -58,13 +59,25 @@ FULL_GRAD_KEYS = (
     "vision_model.embeddings.patch_embedding.weight", "vision_model.embeddings.position_embedding.weight",
     "text_model.encoder.layers.0.mlp.fc1.weight", "text_model.encoder.layers.11.self_attn.q_proj.weight",
     "visual_projection.weight", "text_projection.weight",
+    "vision_model.encoder.layers.0.mlp.fc1.weight", "vision_model.encoder.layers.0.mlp.fc2.weight",
 )
-ROW_GRAD_KEYS = {"vision_model.encoder.layers.0.mlp.fc1.weight": 512, "vision_model.encoder.layers.0.mlp.fc2.weight": 128}
+GRAD_SAMPLES = 4096
 
 
 def _pack_f16(g):
     s = float(g.abs().max().clamp_min(1e-30))
     return {"scale": s, "data": (g / s).to(torch.float16)}
+
+
+def _sample_f16(g, candidates, gen):
+    """Flat indices of g drawn from `candidates` ([rows, width] of flat indices): its first and last row whole, so that a fault
+    confined to an edge tile shows, plus a seeded random pick of the other rows' elements that brings the total to GRAD_SAMPLES
+    (at least GRAD_SAMPLES // 4 of them).  Sorted, with g's values there packed by _pack_f16."""
+    edge = torch.cat([candidates[0], candidates[-1]])
+    inner = candidates[1:-1].flatten()
+    n = max(GRAD_SAMPLES - edge.numel(), GRAD_SAMPLES // 4)
+    pick = torch.cat([edge, inner[torch.randperm(inner.numel(), generator=gen)[:n]]]).sort().values
+    return {"index": pick.to(torch.int32), **_pack_f16(g.flatten()[pick])}
 
 
 def run_case(name, cfg, B, T, Lt, ragged, weight_seed, data_seed, with_hidden, full_grads=False):
@@ -115,17 +128,18 @@ def run_case(name, cfg, B, T, Lt, ragged, weight_seed, data_seed, with_hidden, f
                                                  "vision_model.embeddings.position_embedding"))},
     }
     if full_grads:
-        full = {k: _pack_f16(grads[k]) for k in FULL_GRAD_KEYS}
-        for k, n in ROW_GRAD_KEYS.items():
-            full[k + f"[:{n}]"] = _pack_f16(grads[k][:n])
+        gen = torch.Generator().manual_seed(2024)
+        full = {k: _sample_f16(grads[k], torch.arange(grads[k].numel()).view(grads[k].shape[0], -1), gen)
+                for k in FULL_GRAD_KEYS}
         tk = "text_model.embeddings.token_embedding.weight"
         rows = torch.unique(ids)
-        full[tk + "[rows]"] = {"rows": rows, **_pack_f16(grads[tk][rows])}
+        width = grads[tk].shape[1]
+        full[tk] = _sample_f16(grads[tk], rows[:, None] * width + torch.arange(width), gen)   # touched rows only
         rest = grads[tk].clone()
         rest[rows] = 0
         assert float(rest.abs().max()) == 0.0                                        # untouched rows: exactly zero
         gold["grad_full"] = full
-        gold["grad_vectors"] = {k: g.clone() for k, g in grads.items() if g.dim() <= 1 or g.numel() <= 4096}
+        gold["grad_vectors"] = {k: _pack_f16(g) for k, g in grads.items() if g.dim() <= 1 or g.numel() <= 4096}
     if with_hidden:
         vh = out["vision_model_output"].hidden_states
         th = out["text_model_output"].hidden_states

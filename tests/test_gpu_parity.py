@@ -111,21 +111,15 @@ def _unpack(e):
 
 
 def _errors_vs_full_golden(gold, vis, txt, loss, grads):
-    """Full-tensor relative L2 errors against the fp32 reference golden (features, logits, loss, every kept gradient)."""
+    """Relative L2 errors against the fp32 reference golden (features, logits, loss, every kept gradient: the stored sample of
+    each weight gradient, every bias / LayerNorm gradient vector whole)."""
     e = {"vis": _rel(vis, gold["vis_features"]), "txt": _rel(txt, gold["text_features"]),
          "logits": _rel(vis @ txt.t(), gold["vis_features"] @ gold["text_features"].t()),
          "loss": abs(loss - float(gold["loss"])) / abs(float(gold["loss"]))}
     for k, ent in gold["grad_full"].items():
-        want = _unpack(ent)
-        if k.endswith("[rows]"):
-            got = grads[k[:-6]][ent["rows"]]
-        elif "[:" in k:
-            name, n = k[:k.index("[:")], int(k[k.index("[:") + 2:-1])
-            got = grads[name][:n]
-        else:
-            got = grads[k]
-        e["d " + k] = _rel(got, want)
-    vec = [(k, g) for k, g in gold["grad_vectors"].items() if float(g.norm()) > 1e-3 * gold["grad_norms"]["logit_scale"] and "k_proj.bias" not in k]
+        e["d " + k] = _rel(grads[k].flatten()[ent["index"].long()], _unpack(ent))
+    vectors = {k: _unpack(ent) for k, ent in gold["grad_vectors"].items()}
+    vec = [(k, g) for k, g in vectors.items() if float(g.norm()) > 1e-3 * gold["grad_norms"]["logit_scale"] and "k_proj.bias" not in k]
     e["d vectors (worst)"] = max(_rel(grads[k], g) for k, g in vec)
     e["d vectors (median)"] = sorted(_rel(grads[k], g) for k, g in vec)[len(vec) // 2]
     return e
@@ -136,8 +130,9 @@ CALIBRATION = 1.5      # ours may deviate from the fp32 reference by at most 1.5
 
 def _full12_case(dev, golden_dir, pad_to):
     """T = 12, 12 + 12 layers, ragged text — the BENCH model — against the golden made from the real reference
-    (tests/golden/make_golden.py full12): full-tensor relative L2 of the features, the logits matrix and twelve whole
-    weight-gradient tensors (+ all bias / LayerNorm gradient vectors), each CALIBRATED against the deviation the reference
+    (tests/golden/make_golden.py full12): full-tensor relative L2 of the features and the logits matrix, relative L2 over
+    at least 4096 elements of each of fifteen weight-gradient tensors (first and last row whole, the rest a fixed, seeded
+    sample) and over every bias / LayerNorm gradient vector whole, each CALIBRATED against the deviation the reference
     algorithm itself shows in bf16 on the same inputs on this GPU (autocast and all-bf16), not against a hand-set number.
     With pad_to = 64 the golden batch occupies rows 0..3 of a 64-pair batch (BASELINE.json configs[1]'s per-GPU batch):
     the loss is taken on those rows only, so every gradient must still equal the reference's."""
@@ -175,7 +170,7 @@ def _full12_case(dev, golden_dir, pad_to):
 
 
 def _assert_calibrated(ours, ref):
-    """Full tensors (features, logits matrix, whole gradient tensors): our deviation from the fp32 reference golden may be at
+    """Features, logits matrix and the stored gradients: our deviation from the fp32 reference golden may be at
     most CALIBRATION = 1.5 x the deviation of the REFERENCE's own bf16 path (autocast: fp32 residual stream, bf16 matmul inputs)
     on the same inputs on this GPU — tighter than SURVEY.md §8c's 2x.  Measured (profiles/r02_pytest_gpu_parity_v2_fp32_residual.log):
     features 0.95x, logits 1.24x, gradients 0.93x - 1.29x.  With `residual_fp32=False` (round-1 bf16 stream) the features sit at

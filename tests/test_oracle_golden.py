@@ -268,10 +268,11 @@ def test_swin3d_flop_and_parameter_model_matches_baseline_md():
 
 @pytest.mark.timeout(900)
 def test_full_depth_t12_golden_with_whole_gradient_tensors(golden_dir):
-    """The BENCH model (12 + 12 layers, T = 12, ragged text) with the full gradient tensors the GPU parity test is calibrated
-    on (tests/golden/make_golden.py full12, made from the real reference modules): the oracle replays features, loss, the twelve
-    whole weight-gradient tensors (stored as fp16 after max-normalisation: 2^-11 per element) and every bias / LayerNorm
-    gradient vector in fp32 on the CPU."""
+    """The BENCH model (12 + 12 layers, T = 12, ragged text) with the gradients the GPU parity test is calibrated on
+    (tests/golden/make_golden.py full12, made from the real reference modules): the oracle replays features, loss, at
+    least 4096 elements of each of fifteen weight-gradient tensors (first and last row whole, the rest a fixed, seeded
+    sample) and every bias / LayerNorm gradient vector whole (both stored as fp16 after max-normalisation: 2^-11 per
+    element) in fp32 on the CPU."""
     gold = torch.load(os.path.join(golden_dir, "full12_b4_t12_ragged.pt"), weights_only=False)
     meta = gold["meta"]
     cfg = O.ClipVipCfg()
@@ -289,15 +290,10 @@ def test_full_depth_t12_golden_with_whole_gradient_tensors(golden_dir):
     assert len(gold["grad_full"]) >= 12
     for k, ent in gold["grad_full"].items():
         want = ent["data"].float() * ent["scale"]
-        if k.endswith("[rows]"):
-            got = sd[k[:-6]].grad[ent["rows"]]
-        elif "[:" in k:
-            name, n = k[:k.index("[:")], int(k[k.index("[:") + 2:-1])
-            got = sd[name].grad[:n]
-        else:
-            got = sd[k].grad
+        got = sd[k].grad.flatten()[ent["index"].long()]
         assert _rel(got, want) < 1e-3, (k, _rel(got, want))       # fp16 storage of the golden: ~3e-4
     ref_norm = gold["grad_norms"]["logit_scale"]
-    for k, g in gold["grad_vectors"].items():
+    for k, ent in gold["grad_vectors"].items():
+        g = ent["data"].float() * ent["scale"]
         if float(g.norm()) > 1e-3 * ref_norm:
             assert _rel(sd[k].grad, g) < 1e-3, (k, _rel(sd[k].grad, g))
